@@ -7,6 +7,17 @@ bench.py -- BASELINE.json's metric: voxels/s warped (SpatialTransformer / interp
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...                           # CPU port of the reference, host cores
     python bench.py --op dice|cce|lc3d|resize|warp_mc|warp_slab|cfg5|mi|mi_segs|blur ...   # one op per line
+    python bench.py ... --dump-outputs DIR                         # + DIR/<name>.npy: the last timed step's output
+
+The inputs are drawn from fixed seeds, so two builds run with the same arguments can be compared output for output
+through --dump-outputs.  Every record that runs a timed step writes one array: the headline warp as warp.npy, the
+default line's ops as dice, cce, lc3d, lc3d_b8, resize and warp_c16, its N-GPU records as slab, slab_c16, cfg5_batch and
+cfg5_slab, and the --op lines under their own names (mi, mi_segs, blur, slab / slab_c<C>, lc3d_b<B>, warp_c<C>, ...).
+At N GPUs, rank 0 writes what it computed: its own batch, or its planes of a z-slab-sharded volume.  --impl reference
+runs no GPU step and writes nothing.
+
+Step counts: --steps sets the timed steps of the line's own measurement, --long-steps those of the headline's long_run
+and of every sub-record of the default line, --e2e-steps and --cfg5-steps those of the e2e and cfg5 records.
 
 A "step" is one pass of the hot path over one batch: `--batch` (default 8) independent
 160x192x224x1 volumes with a random dense 3-channel flow U(-3,3) (configs[1] of
@@ -20,7 +31,7 @@ JSON keys beyond the base contract:
   roofline     achieved = 20 B/voxel (12 flow + 4 source-once + 4 store, SURVEY.md 8d)
                * voxels per launch / launch time; peak = MEASURED_PEAKS.json hbm_gbs.
                `traffic` is the ncu dram__bytes of the committed capture (profiles/traffic.json, static).
-  long_run     the same launch timed over >= 200 steps (the K steps of the contract are only a few ms)
+  long_run     the same launch timed over --long-steps steps (default 200; K steps of a short run are only a few ms)
   e2e          the same metric through the public API with HOST (pinned) buffers: H2D of
                vol+flow and D2H of the result inside the timed region, every step.
   cpu_baseline the oracle's C/OpenMP port on the host cores, bounded sample (rank 0, N=1), MEDIAN of >= 20 runs
@@ -44,7 +55,6 @@ sys.path.insert(0, ROOT)
 
 SHAPE = (160, 192, 224)
 V = SHAPE[0] * SHAPE[1] * SHAPE[2]
-OPS_STEPS = 200
 
 
 def measured_peak():
@@ -192,10 +202,10 @@ def dist_setup(n_gpus):
     return world, rank, local
 
 
-def timed_region(fn, steps, warmup, world, min_preheat_s=0.3):
+def timed_region(fn, steps, warmup, world, min_preheat_s=0.3, last=None):
     """W warm-up steps, then exactly K steps between CUDA events, barrier + sync both sides,
     max over ranks.  A short pre-heat (not counted) lets the clocks settle and gives the
-    sampler something to see."""
+    sampler something to see.  If `last` is a list, what the K-th timed call returned is appended to it."""
     import torch
     import torch.distributed as dist
     if world > 1:
@@ -217,15 +227,36 @@ def timed_region(fn, steps, warmup, world, min_preheat_s=0.3):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(steps):
-        fn()
+        out = fn()
     e1.record()
     torch.cuda.synchronize()
+    ms = e0.elapsed_time(e1)
     if world > 1:
         dist.barrier()
-    ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device='cuda')
-    if world > 1:
-        dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-    return float(ms.item())
+        t = torch.tensor([ms], dtype=torch.float64, device='cuda')
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+        ms = t.item()
+    if last is not None and steps > 0:
+        last.append(out)
+    return float(ms)
+
+
+DUMP_ELEMS = 1 << 21          # 8 MB of float32 per array; a line dumps at most 7 arrays, under 64 MB in all
+
+
+def dump_output(args, name, last, rank=0):
+    """--dump-outputs DIR: what the last timed step returned, as DIR/<name>.npy in float32.  An output of more than
+    DUMP_ELEMS elements is sampled at DUMP_ELEMS flat indices drawn from a fixed seed, the same in every run."""
+    if not args.dump_outputs or rank != 0:
+        return
+    import numpy as np
+    import torch
+    out = last[-1].detach().reshape(-1)
+    if out.numel() > DUMP_ELEMS:
+        idx = np.sort(np.random.default_rng(0).choice(out.numel(), DUMP_ELEMS, replace=False))
+        out = out[torch.from_numpy(idx).to(out.device)]
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    np.save(os.path.join(args.dump_outputs, name + '.npy'), out.float().cpu().numpy())
 
 
 # ---------------------------------------------------------------------------------------
@@ -340,25 +371,19 @@ def bench_reference(args):
     warm = max(args.warmup, 3)
     for _ in range(warm):
         fn()
-    steps = max(1, min(args.steps, 200))
+    steps = args.steps
     ts = []
     for _ in range(steps):
         t = time.time()
         fn()
         ts.append(time.time() - t)
-    extra = 0
-    while len(ts) < 20:                                      # the statistic needs >= 20 runs even if K is small
-        t = time.time()
-        fn()
-        ts.append(time.time() - t)
-        extra += 1
     ts.sort()
     med = ts[len(ts) // 2]
     value = V / med
     sample = ('each step = ONE 160x192x224 volume (bounded sample of the batch-%d step), oracle/c C99+OpenMP port, '
-              '%d threads bound to cores, inputs first-touched by the OpenMP threads; value = V / MEDIAN step time over %d '
-              'runs (%d steps + %d extra for the statistic; best %.3g, worst %.3g voxels/s)'
-              % (args.batch, cport.num_threads(), len(ts), steps, extra, V / ts[0], V / ts[-1]))
+              '%d threads bound to cores, inputs first-touched by the OpenMP threads; value = V / MEDIAN step time over the '
+              '%d steps (best %.3g, worst %.3g voxels/s)'
+              % (args.batch, cport.num_threads(), steps, V / ts[0], V / ts[-1]))
     print(json.dumps({
         'impl': 'reference',
         'metric': 'voxels/s warped (SpatialTransformer / interpn %s), 160x192x224 fp32' % args.method,
@@ -393,8 +418,9 @@ def bench_warp(args):
         flow = (flow / flow.abs().amax() * 8).permute(0, 2, 3, 4, 1).contiguous()
     st = ne.layers.SpatialTransformer(interp_method=args.method, fill_value=None, halo=args.halo)
     sampler = ClockSampler(local).start()
-    ms = timed_region(lambda: st([vol, flow]), args.steps, args.warmup, world)
-    long_steps = max(args.steps, OPS_STEPS)
+    last = []
+    ms = timed_region(lambda: st([vol, flow]), args.steps, args.warmup, world, last=last)
+    long_steps = args.long_steps
     ms_long = timed_region(lambda: st([vol, flow]), long_steps, 3, world, min_preheat_s=0.0)
     clocks = sampler.stop()
     vox_per_step = world * B * V
@@ -402,7 +428,7 @@ def bench_warp(args):
     bytes_per_launch = 20.0 * B * V
 
     # ---- end to end through the public API with host buffers (pinned, allocated after the NUMA binding)
-    e2e_steps = max(1, min(args.steps, args.e2e_steps))
+    e2e_steps = args.e2e_steps
     h_vol = torch.empty(vol.shape, dtype=torch.float32).pin_memory().copy_(vol.cpu())
     h_flow = torch.empty(flow.shape, dtype=torch.float32).pin_memory().copy_(flow.cpu())
     h_out = torch.empty(vol.shape, dtype=torch.float32).pin_memory()
@@ -433,7 +459,9 @@ def bench_warp(args):
         'gpu_launches': args.steps,
         'clocks': clocks,
     }
-    del vol, flow
+    # written after every timed region of the headline, so that the copy-out cannot disturb them
+    dump_output(args, 'warp', last, rank)
+    del vol, flow, last
     torch.cuda.empty_cache()
     # the NUMA binding was for the pinned staging buffers of the end-to-end path; the CPU legs below use every core
     if orig_aff:
@@ -445,9 +473,9 @@ def bench_warp(args):
         if world == 1:
             line['ops'] = run_ops(args, world, rank, local, dev)
         else:
-            for key, fn in (('slab', lambda: slab_record(args, world, rank, dev, channels=1, batch=1)),
-                            ('slab_c16', lambda: slab_record(args, world, rank, dev, channels=16, batch=1)),
-                            ('cfg5', lambda: cfg5_record(args, world, rank, dev))):
+            for key, fn in (('slab', lambda: slab_record(args, world, rank, dev, args.long_steps, channels=1, batch=1)),
+                            ('slab_c16', lambda: slab_record(args, world, rank, dev, args.long_steps, channels=16, batch=1)),
+                            ('cfg5', lambda: cfg5_record(args, world, rank, dev, args.cfg5_steps))):
                 try:
                     line[key] = fn()
                 except Exception as ex:                      # noqa: BLE001 -- a sub-record must not take the headline down
@@ -465,12 +493,13 @@ def bench_warp(args):
 def run_ops(args, world, rank, local, dev):
     """The other BASELINE.json configs inside the default line (driver-visible): compact records."""
     ops = {}
-    for name, fn in (('dice', lambda: dice_record(args, world, rank, dev, cce=False)),
-                     ('cce', lambda: dice_record(args, world, rank, dev, cce=True)),
-                     ('lc3d', lambda: lc3d_record(args, world, rank, dev, batch=1)),
-                     ('lc3d_b8', lambda: lc3d_record(args, world, rank, dev, batch=8, cpu=False)),
-                     ('resize', lambda: resize_record(args, world, rank, dev)),
-                     ('warp_c16', lambda: warp_mc_record(args, world, rank, dev, 16))):
+    steps = args.long_steps
+    for name, fn in (('dice', lambda: dice_record(args, world, rank, dev, steps, cce=False)),
+                     ('cce', lambda: dice_record(args, world, rank, dev, steps, cce=True)),
+                     ('lc3d', lambda: lc3d_record(args, world, rank, dev, steps, batch=1)),
+                     ('lc3d_b8', lambda: lc3d_record(args, world, rank, dev, steps, batch=8, cpu=False)),
+                     ('resize', lambda: resize_record(args, world, rank, dev, steps)),
+                     ('warp_c16', lambda: warp_mc_record(args, world, rank, dev, steps, 16))):
         try:
             r = fn()
             ops[name] = {'workload': r['config']['workload'], 'metric': r['metric'], 'value': r['value'], 'unit': r['unit'],
@@ -495,13 +524,12 @@ def base_line(metric, value, unit, world, steps, warmup, ms, scaling, workload, 
             'data': 'synthetic', 'config': cfg}
 
 
-def dice_record(args, world, rank, dev, cce=False):
+def dice_record(args, world, rank, dev, steps, cce=False):
     import numpy as np
     import torch
     import neurite_b200 as ne
     from neurite_b200.dist import slab_bounds
     B, L = 4, 16
-    steps = max(args.steps, OPS_STEPS)
     # cfg 3: batch 4 < 8 GPUs -> shard the voxel range of every batch item across ranks (strong scaling)
     z0, nz = slab_bounds(SHAPE[0], world, rank)
     g = torch.Generator(device=dev).manual_seed(7 + rank)
@@ -511,8 +539,10 @@ def dice_record(args, world, rank, dev, cce=False):
     group = torch.distributed.group.WORLD if world > 1 else None
     op = ne.losses.CategoricalCrossentropy(group=group) if cce else ne.losses.Dice(group=group)
     sampler = ClockSampler(dev.index).start()
-    ms = timed_region(lambda: op.loss(t, p), steps, args.warmup, world)
+    last = []
+    ms = timed_region(lambda: op.loss(t, p), steps, args.warmup, world, last=last)
     clocks = sampler.stop()
+    dump_output(args, 'cce' if cce else 'dice', last, rank)
     elems = B * V * L
     name = 'CategoricalCrossentropy' if cce else 'Dice().loss'
     line = base_line('(voxel,label) elements/s, %s on 16-label one-hot 160x192x224, batch 4' % ('CCE' if cce else 'Dice loss'),
@@ -538,12 +568,11 @@ def dice_record(args, world, rank, dev, cce=False):
     return line
 
 
-def lc3d_record(args, world, rank, dev, batch=None, cpu=True):
+def lc3d_record(args, world, rank, dev, steps, batch=None, cpu=True):
     import numpy as np
     import torch
     from neurite_b200.layers import local_conv3d
     B = batch or args.lc_batch
-    steps = max(args.steps, OPS_STEPS)
     I, Cin, Cout = 64, 16, 16
     O = I - 2
     P, F = O ** 3, 27 * Cin
@@ -553,8 +582,11 @@ def lc3d_record(args, world, rank, dev, batch=None, cpu=True):
     kernel = (torch.rand((P, F, Cout), device=dev, generator=g) * 2 - 1) * lim
     bias = torch.randn((O, O, O, Cout), device=dev, generator=g)
     sampler = ClockSampler(dev.index).start()
-    ms = timed_region(lambda: local_conv3d(x, kernel, bias, (3, 3, 3), (1, 1, 1), (O, O, O)), steps, args.warmup, world)
+    last = []
+    ms = timed_region(lambda: local_conv3d(x, kernel, bias, (3, 3, 3), (1, 1, 1), (O, O, O)), steps, args.warmup, world,
+                      last=last)
     clocks = sampler.stop()
+    dump_output(args, 'lc3d' if B == 1 else 'lc3d_b%d' % B, last, rank)
     line = base_line('output positions/s, LocallyConnected3D 3^3 16->16 on 64^3, batch %d' % B,
                      P * B * steps / (ms * 1e-3), 'positions/s', world, steps, args.warmup, ms, 'weak',
                      'BASELINE.json configs[3]: LocallyConnected3D 3x3x3, 16->16, input [%d,64,64,64,16], kernel '
@@ -579,17 +611,19 @@ def lc3d_record(args, world, rank, dev, batch=None, cpu=True):
     return line
 
 
-def resize_record(args, world, rank, dev):
+def resize_record(args, world, rank, dev, steps):
     import numpy as np
     import torch
     import neurite_b200 as ne
     B = args.batch
-    steps = max(args.steps, OPS_STEPS)
-    x = torch.randn((B, 80, 96, 112, 3), device=dev)
+    g = torch.Generator(device=dev).manual_seed(5 + rank)
+    x = torch.randn((B, 80, 96, 112, 3), device=dev, generator=g)
     lay = ne.layers.Resize(2)
     sampler = ClockSampler(dev.index).start()
-    ms = timed_region(lambda: lay(x), steps, args.warmup, world)
+    last = []
+    ms = timed_region(lambda: lay(x), steps, args.warmup, world, last=last)
     clocks = sampler.stop()
+    dump_output(args, 'resize', last, rank)
     line = base_line('output voxels/s, Resize zoom 2 of a half-resolution 3-ch flow to 160x192x224',
                      world * B * V * steps / (ms * 1e-3), 'voxels/s', world, steps, args.warmup, ms, 'weak',
                      'Resize(2) on [%d,80,96,112,3] (reference models.py:803-804)' % B)
@@ -612,7 +646,7 @@ def resize_record(args, world, rank, dev):
     return line
 
 
-def warp_mc_record(args, world, rank, dev, C=None):
+def warp_mc_record(args, world, rank, dev, steps, C=None):
     """Multi-channel warp (the kernel of BASELINE.json configs[4]: a 16-label softmax through the
     SpatialTransformer): z-marching ring kernel, (12 + 8C) B per voxel."""
     import numpy as np
@@ -620,7 +654,6 @@ def warp_mc_record(args, world, rank, dev, C=None):
     import neurite_b200 as ne
     C = C or args.channels
     B = max(1, min(args.batch, 32 // C))
-    steps = max(args.steps, 50)
     g = torch.Generator(device=dev).manual_seed(11 + rank)
     vol = torch.randn((B,) + SHAPE + (C,), device=dev, generator=g)
     flow = torch.rand((B,) + SHAPE + (3,), device=dev, generator=g) * 6 - 3
@@ -630,8 +663,10 @@ def warp_mc_record(args, world, rank, dev, C=None):
         flow = (flow / flow.abs().amax() * 3).permute(0, 2, 3, 4, 1).contiguous()
     st = ne.layers.SpatialTransformer(interp_method=args.method)
     sampler = ClockSampler(dev.index).start()
-    ms = timed_region(lambda: st([vol, flow]), steps, args.warmup, world)
+    last = []
+    ms = timed_region(lambda: st([vol, flow]), steps, args.warmup, world, last=last)
     clocks = sampler.stop()
+    dump_output(args, 'warp_c%d' % C, last, rank)
     line = base_line('voxels/s warped, %d-channel volume (SpatialTransformer %s)' % (C, args.method),
                      world * B * V * steps / (ms * 1e-3), 'voxels/s', world, steps, args.warmup, ms, 'weak',
                      'SpatialTransformer warp of [%d,160,192,224,%d] fp32 (the %d-label softmax of BASELINE.json configs[4]), '
@@ -655,12 +690,11 @@ def warp_mc_record(args, world, rank, dev, C=None):
 # ---------------------------------------------------------------------------------------
 # ONE volume over N ranks: z-slabs + halo exchange (strong scaling, SURVEY.md 8e)
 # ---------------------------------------------------------------------------------------
-def slab_record(args, world, rank, dev, channels=1, batch=1):
+def slab_record(args, world, rank, dev, steps, channels=1, batch=1):
     import torch
     import torch.distributed as dist
     from neurite_b200 import dist as nd, utils
     C, B = channels, batch
-    steps = max(args.steps, OPS_STEPS)
     g = torch.Generator(device=dev).manual_seed(77)          # every rank draws the same volume and keeps its planes
     z0, nz = nd.slab_bounds(SHAPE[0], world, rank)
     vol = torch.randn((B,) + SHAPE + (C,), device=dev, generator=g)[:, z0:z0 + nz].contiguous()
@@ -671,9 +705,11 @@ def slab_record(args, world, rank, dev, channels=1, batch=1):
                        'U(-3,3) i.i.d., halo %d planes from each neighbour' % (B, C, world, nz, halo),
            'scaling': 'strong', 'n_gpus': world, 'steps': steps, 'halo_planes': halo,
            'halo_bytes_per_rank_per_step': int(2 * halo * SHAPE[1] * SHAPE[2] * C * 4 * B)}
+    name = 'slab' if C == 1 else 'slab_c%d' % C
     if world == 1:
         out = torch.empty_like(vol)
         ms = timed_region(lambda: utils._warp_views(vol, flow, out, SHAPE[0], 0, None, 0, 0), steps, 3, world)
+        dump_output(args, name, [out], rank)               # every step overwrites `out`: it holds the last one
         rec['overlap'] = {'ms_per_step': ms / steps, 'value': B * V * steps / (ms * 1e-3), 'unit': 'voxels/s'}
         return rec
     out = torch.empty(tuple(flow.shape[:-1]) + (C,), dtype=torch.float32, device=dev)
@@ -686,6 +722,8 @@ def slab_record(args, world, rank, dev, channels=1, batch=1):
         src = plan.source_view(vol)
         src.copy_(vol)
         ms_ov = timed_region(lambda: plan(src, flow, out), steps, 3, world, min_preheat_s=0.1)
+        if transport == 'auto':
+            dump_output(args, name, [out], rank)           # rank 0's planes of the last step
         plan.check()
         # the two ingredients on their own: the halo exchange (no kernels) and the three launches (no exchange)
         ext, pad = plan._buffers(vol), plan._pad
@@ -730,27 +768,27 @@ def slab_record(args, world, rank, dev, channels=1, batch=1):
                               'nccl = one ncclGroup of send/recv')
     if rec['overlap']['transport'] == 'peer':
         rec['overlap_nccl'] = measure('nccl')
-    ser_steps = max(20, steps // 4)
+    ser_steps = max(1, steps // 4)
     ms_ser = timed_region(lambda: nd.warp_slab(vol, flow, SHAPE[0], mode='serial', halo=halo), ser_steps, 3, world, min_preheat_s=0.0)
-    rec['serial'] = {'ms_per_step': ms_ser / ser_steps, 'value': B * V * ser_steps / (ms_ser * 1e-3), 'unit': 'voxels/s',
+    rec['serial'] = {'steps': ser_steps, 'ms_per_step': ms_ser / ser_steps, 'value': B * V * ser_steps / (ms_ser * 1e-3), 'unit': 'voxels/s',
                      'what': 'round-1 path: NCCL exchange, then one launch, err.item() every step'}
     # strong-scaling reference: the same batch on ONE GPU (no exchange), timed on rank 0's device
     g1 = torch.Generator(device=dev).manual_seed(78)
     vol1 = torch.randn((B,) + SHAPE + (C,), device=dev, generator=g1)
     flow1 = torch.rand((B,) + SHAPE + (3,), device=dev, generator=g1) * 6 - 3
     out1 = torch.empty_like(vol1)
-    ms_one = timed_region(lambda: utils._warp_views(vol1, flow1, out1, SHAPE[0], 0, None, 0, 0), max(20, steps // 4), 3, world,
+    ms_one = timed_region(lambda: utils._warp_views(vol1, flow1, out1, SHAPE[0], 0, None, 0, 0), ser_steps, 3, world,
                           min_preheat_s=0.0)
     best = rec['overlap']['ms_per_step']
     gr = rec['overlap'].get('cuda_graph_replay') or {}
     if 'ms_per_step' in gr:
         best = min(best, gr['ms_per_step'])
-    rec['one_gpu_whole_volume'] = {'ms_per_step': ms_one / max(20, steps // 4),
-                                   'speedup_of_the_slab_plan': (ms_one / max(20, steps // 4)) / best}
+    rec['one_gpu_whole_volume'] = {'ms_per_step': ms_one / ser_steps, 'steps': ser_steps,
+                                   'speedup_of_the_slab_plan': (ms_one / ser_steps) / best}
     return rec
 
 
-def cfg5_record(args, world, rank, dev):
+def cfg5_record(args, world, rank, dev, steps):
     """BASELINE.json configs[4]: UNet fwd -> SpatialTransformer (16 labels) -> Dice, global batch = N volumes
     (one per GPU), batch-sharded and z-slab-sharded.  The UNet is stock torch/cuDNN (context); the warp and the Dice
     are this repo's kernels and are the part that counts toward the roofline."""
@@ -759,7 +797,6 @@ def cfg5_record(args, world, rank, dev):
     ex = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(ex)
     group = torch.distributed.group.WORLD if world > 1 else None
-    steps = max(3, min(args.cfg5_steps, 50))
     rec = {'workload': 'UNet(16 features, 4 levels, bf16 autocast, cuDNN) fwd -> SpatialTransformer of the 16-label softmax -> '
                        'Dice vs one-hot target, 160x192x224, global batch %d' % max(world, args.cfg5_batch),
            'n_gpus': world, 'steps': steps}
@@ -782,7 +819,9 @@ def cfg5_record(args, world, rank, dev):
             e.record()
             evs.append(e)
             return job.step(mark)
-        ms = timed_region(lambda: job.step(), steps, 2, world, min_preheat_s=0.0)
+        last = []
+        ms = timed_region(lambda: job.step(), steps, 2, world, min_preheat_s=0.0, last=last)
+        dump_output(args, 'cfg5_' + mode, last, rank)
         loss = job.step()
         evs.clear()
         for _ in range(3):
@@ -827,19 +866,22 @@ def bench_mi(args, segs=False):
     world, rank, local = dist_setup(args.gpus)
     dev = torch.device('cuda', local)
     m = ne.metrics.MutualInformation(nb_bins=16)
+    g = torch.Generator(device=dev).manual_seed(13 + rank)
     if segs:
         B = 2
-        x = torch.softmax(torch.randn((B,) + SHAPE + (16,), device=dev), -1)
-        y = torch.softmax(torch.randn((B,) + SHAPE + (16,), device=dev), -1)
+        x = torch.softmax(torch.randn((B,) + SHAPE + (16,), device=dev, generator=g), -1)
+        y = torch.softmax(torch.randn((B,) + SHAPE + (16,), device=dev, generator=g), -1)
         fn, per_voxel, kern = (lambda: m.segs(x, y)), 128.0, 'mi_hist_mma_kernel<1,2,maps,maps>'
     else:
         B = args.batch
-        x = torch.rand((B,) + SHAPE + (1,), device=dev)
-        y = (0.7 * x * x + 0.1 + 0.1 * torch.rand_like(x)).clamp_(0, 1)
+        x = torch.rand((B,) + SHAPE + (1,), device=dev, generator=g)
+        y = (0.7 * x * x + 0.1 + 0.1 * torch.rand(x.shape, device=dev, generator=g)).clamp_(0, 1)
         fn, per_voxel, kern = (lambda: m.volumes(x, y)), 8.0, 'mi_hist_mma_kernel<1,2,quant,quant>'
     sampler = ClockSampler(local).start()
-    ms = timed_region(fn, args.steps, args.warmup, world)
+    last = []
+    ms = timed_region(fn, args.steps, args.warmup, world, last=last)
     clocks = sampler.stop()
+    dump_output(args, 'mi_segs' if segs else 'mi', last, rank)
     if rank == 0:
         line = base_line('voxels/s, MutualInformation.%s (16 bins), 160x192x224 fp32' % ('segs' if segs else 'volumes'),
                          world * B * V * args.steps / (ms * 1e-3), 'voxels/s', world, args.steps, args.warmup, ms, 'weak',
@@ -874,11 +916,14 @@ def bench_blur(args):
     world, rank, local = dist_setup(args.gpus)
     dev = torch.device('cuda', local)
     B = args.batch
-    x = torch.randn((B,) + SHAPE + (1,), device=dev)
+    g = torch.Generator(device=dev).manual_seed(17 + rank)
+    x = torch.randn((B,) + SHAPE + (1,), device=dev, generator=g)
     lay = ne.layers.GaussianBlur(sigma=args.sigma)
     sampler = ClockSampler(local).start()
-    ms = timed_region(lambda: lay(x), args.steps, args.warmup, world)
+    last = []
+    ms = timed_region(lambda: lay(x), args.steps, args.warmup, world, last=last)
     clocks = sampler.stop()
+    dump_output(args, 'blur', last, rank)
     if rank == 0:
         line = base_line('voxels/s, GaussianBlur(sigma=%g), 160x192x224 fp32' % args.sigma,
                          world * B * V * args.steps / (ms * 1e-3), 'voxels/s', world, args.steps, args.warmup, ms, 'weak',
@@ -905,7 +950,7 @@ def single_op(args, fn):
     import torch
     world, rank, local = dist_setup(args.gpus)
     dev = torch.device('cuda', local)
-    rec = fn(args, world, rank, dev)
+    rec = fn(args, world, rank, dev, args.steps)
     if rank == 0:
         print(json.dumps(rec), flush=True)
     finish(world)
@@ -921,7 +966,10 @@ def finish(world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=200)
+    ap.add_argument('--steps', type=int, default=200, help='timed steps of the line\'s own measurement')
+    ap.add_argument('--long-steps', type=int, default=200,
+                    help='timed steps of the headline\'s long_run and of each sub-record of the default line '
+                         '(ops at 1 GPU, slab and slab_c16 at N GPUs)')
     ap.add_argument('--warmup', type=int, default=5)
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--op', default='warp', choices=['warp', 'dice', 'cce', 'lc3d', 'resize', 'warp_mc', 'warp_slab', 'cfg5',
@@ -932,15 +980,19 @@ def main():
     ap.add_argument('--lc-batch', type=int, default=1)
     ap.add_argument('--slab-batch', type=int, default=1)
     ap.add_argument('--slab-channels', type=int, default=1)
-    ap.add_argument('--cfg5-steps', type=int, default=5)
+    ap.add_argument('--cfg5-steps', type=int, default=5, help='timed steps of the cfg5 record')
     ap.add_argument('--cfg5-batch', type=int, default=0, help='global batch of --op cfg5 (default: one volume per GPU)')
     ap.add_argument('--method', default='linear', choices=['linear', 'nearest'])
     ap.add_argument('--flow', default='iid', choices=['iid', 'smooth'])
     ap.add_argument('--halo', type=int, default=0)
-    ap.add_argument('--e2e-steps', type=int, default=10)
+    ap.add_argument('--e2e-steps', type=int, default=10, help='timed steps of the headline\'s e2e record')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-numpy-baseline', action='store_true')
     ap.add_argument('--no-extras', action='store_true', help='headline only: no ops / slab / cfg5 sub-records')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last timed step of each record computed as '
+                         'DIR/<name>.npy (float32; outputs over %d elements as a fixed seeded sample; rank 0\'s '
+                         'outputs at N GPUs)' % DUMP_ELEMS)
     args = ap.parse_args()
     if args.impl == 'reference':
         return bench_reference(args)
@@ -955,11 +1007,11 @@ def main():
     if args.op == 'blur':
         return bench_blur(args)
     single_op(args, {
-        'dice': lambda a, w, r, d: dice_record(a, w, r, d, cce=False),
-        'cce': lambda a, w, r, d: dice_record(a, w, r, d, cce=True),
+        'dice': lambda a, w, r, d, k: dice_record(a, w, r, d, k, cce=False),
+        'cce': lambda a, w, r, d, k: dice_record(a, w, r, d, k, cce=True),
         'lc3d': lc3d_record, 'resize': resize_record, 'warp_mc': warp_mc_record,
-        'warp_slab': lambda a, w, r, d: slab_record(a, w, r, d, channels=a.slab_channels, batch=a.slab_batch),
-        'cfg5': cfg5_record}[args.op])
+        'warp_slab': lambda a, w, r, d, k: slab_record(a, w, r, d, k, channels=a.slab_channels, batch=a.slab_batch),
+        'cfg5': lambda a, w, r, d, k: cfg5_record(a, w, r, d, a.cfg5_steps)}[args.op])
 
 
 if __name__ == '__main__':

@@ -96,6 +96,87 @@ def test_reference_arm_and_our_arm_share_one_config():
     assert c['batch_per_gpu'] == 8 and c['volume'] == [160, 192, 224] and 'configs[1]' in c['workload']
 
 
+def test_dump_outputs_writes_the_last_step_and_a_fixed_sample_of_large_outputs(tmp_path):
+    import argparse
+    import torch
+    import bench
+    args = argparse.Namespace(dump_outputs=str(tmp_path / 'dump'))
+    small = torch.arange(10, dtype=torch.float64)
+    big = torch.arange(bench.DUMP_ELEMS + 1000, dtype=torch.float32).reshape(-1, 8)
+    bench.dump_output(args, 'small', [small * 0, small])
+    bench.dump_output(args, 'big', [big])
+    bench.dump_output(args, 'big_again', [big.clone()])
+    bench.dump_output(args, 'other_rank', [small], rank=1)
+    s = np.load(tmp_path / 'dump' / 'small.npy')
+    assert s.dtype == np.float32 and np.array_equal(s, np.arange(10))
+    b = np.load(tmp_path / 'dump' / 'big.npy')
+    assert b.dtype == np.float32 and b.shape == (bench.DUMP_ELEMS,) and np.all(np.diff(b) > 0)
+    assert np.array_equal(b, np.load(tmp_path / 'dump' / 'big_again.npy'))
+    assert not (tmp_path / 'dump' / 'other_rank.npy').exists()
+    bench.dump_output(argparse.Namespace(dump_outputs=None), 'off', [small])
+    assert sorted(os.listdir(tmp_path / 'dump')) == ['big.npy', 'big_again.npy', 'small.npy']
+
+
+def test_timed_region_times_exactly_k_steps_and_hands_over_the_last_output(monkeypatch):
+    import torch
+    import bench
+    calls = []
+
+    class Event:
+        def __init__(self, enable_timing=False):
+            self.at = None
+
+        def record(self):
+            self.at = len(calls)
+
+        def elapsed_time(self, end):
+            return float(end.at - self.at)          # 1 ms per call between the two events
+
+    monkeypatch.setattr(torch.cuda, 'Event', Event)
+    monkeypatch.setattr(torch.cuda, 'synchronize', lambda *a: None)
+
+    def fn():
+        calls.append(1)
+        return len(calls)
+    for steps, warmup in ((7, 5), (1, 0), (0, 4)):
+        calls.clear()
+        last = []
+        ms = bench.timed_region(fn, steps, warmup, 1, min_preheat_s=0.0, last=last)
+        assert ms == steps and len(calls) == max(warmup, 3) + steps
+        assert last == ([len(calls)] if steps else [])
+
+
+def test_step_flags_set_the_steps_of_every_record(monkeypatch, capsys):
+    import argparse
+    import torch
+    import bench
+    seen = {}
+
+    def fake(name):
+        def rec(args, world, rank, dev, steps, *a, **k):
+            key = name + ('_cce' if k.get('cce') else '') + ('_b%d' % k['batch'] if k.get('batch') else '')
+            seen[key] = steps
+            return {'config': {'workload': key}, 'metric': key, 'value': 1.0, 'unit': 'u', 'steps': steps,
+                    'ms_per_step': 1.0, 'gpu_launches': steps,
+                    'roofline': dict.fromkeys(('achieved', 'peak', 'frac', 'bytes_model', 'traffic', 'traffic_source'))}
+        return rec
+    for name in ('dice', 'lc3d', 'resize', 'warp_mc', 'slab', 'cfg5'):
+        monkeypatch.setattr(bench, name + '_record', fake(name))
+    # the default line's sub-records follow --long-steps
+    bench.run_ops(argparse.Namespace(long_steps=13), 1, 0, 0, torch.device('cpu'))
+    assert seen == {'dice': 13, 'dice_cce': 13, 'lc3d_b1': 13, 'lc3d_b8': 13, 'resize': 13, 'warp_mc': 13}
+    # an --op line times --steps (cfg5: --cfg5-steps)
+    monkeypatch.setattr(torch.cuda, 'is_available', lambda: True)
+    monkeypatch.setattr(bench, 'dist_setup', lambda n: (1, 0, 0))
+    for op, key in (('dice', 'dice'), ('cce', 'dice_cce'), ('lc3d', 'lc3d'), ('resize', 'resize'), ('warp_mc', 'warp_mc'),
+                    ('warp_slab', 'slab_b1'), ('cfg5', 'cfg5')):
+        seen.clear()
+        monkeypatch.setattr(sys, 'argv', ['bench.py', '--op', op, '--steps', '7', '--cfg5-steps', '4'])
+        bench.main()
+        assert seen == {key: 4 if op == 'cfg5' else 7}
+        assert json.loads(capsys.readouterr().out.strip().splitlines()[-1])['steps'] == seen[key]
+
+
 def test_gpu_arm_refuses_to_run_without_a_device():
     import torch
     if torch.cuda.is_available():
